@@ -5,6 +5,7 @@
     python -m torch.distributed.run --nnodes=1 --nproc-per-node N --master-addr 127.0.0.1 --master-port P \
         bench.py --gpus N --steps K --warmup W
     python bench.py --impl reference ...       # the UNMODIFIED reference's generate() on the host cores
+    python bench.py ... --dump-outputs DIR     # also write the last timed step's outputs as DIR/*.npy (compare two builds)
 
 One "step" = one full pass of the hot path (conditioning network + all T*hop autoregressive sample steps + mu-law
 decode/fade) over this rank's batch of synthetic 80-frame mels, on the SHIPPED checkpoint when its travel copy is present
@@ -37,7 +38,7 @@ STEP_WEIGHT_BYTES = 17_371_136          # all per-step weights + biases, fp32, t
 COND_BYTES_PER_UTT = 836                # 80 mel + 128 aux fp32 in, 4 B out, per utterance-sample
 FLOP_PER_SAMPLE = 8_668_160             # 2 * 4 334 080 MAC per utterance-sample
 CKPT_TRAVEL = os.path.join(ROOT, 'oracle', '_ref', 'latest_weights.pyt')
-CKPT_CONTAINER = '/root/reference/logs_wavernn/checkpoints/latest_weights.pyt'
+DUMP_BUDGET = 64_000_000                # bytes --dump-outputs may write in all
 
 
 def parse():
@@ -56,7 +57,32 @@ def parse():
     ap.add_argument('--no-strong', action='store_true', help='skip the strong-scaling (global batch) measurement')
     ap.add_argument('--no-cpu-baseline', action='store_true')
     ap.add_argument('--no-e2e', action='store_true')
-    return ap.parse_args()
+    ap.add_argument('--dump-outputs', metavar='DIR', default=None,
+                    help='after the timed steps, write what the last timed step computed as DIR/<name>.npy (float32 or float64, '
+                         'at most 64 MB in all: larger outputs keep a fixed, seeded sample of their rows, listed in <name>_rows.npy)')
+    args = ap.parse_args()
+    if args.steps < 1 or args.warmup < 0:
+        ap.error('--steps must be >= 1 and --warmup >= 0')
+    if args.dump_outputs and args.impl == 'reference':
+        ap.error('--dump-outputs: the reference arm only times bounded samples of its loop')
+    return args
+
+
+def dump_outputs(path, arrays):
+    """Writes each array as path/<name>.npy: float64 stays float64, every other dtype becomes float32 (exact for the int16
+    labels).  When they would exceed DUMP_BUDGET bytes together, each keeps the same fraction of its rows (axis 0), chosen
+    with a fixed seed and recorded in <name>_rows.npy, so that the same arguments always dump the same elements."""
+    os.makedirs(path, exist_ok=True)
+    arrays = {k: np.asarray(v.cpu() if hasattr(v, 'cpu') else v) for k, v in arrays.items()}
+    arrays = {k: v if v.dtype == np.float64 else v.astype(np.float32) for k, v in arrays.items()}
+    need = sum(v.nbytes + 8 * len(v) + 256 for v in arrays.values())          # + row indices and .npy headers
+    frac = min(1.0, DUMP_BUDGET / need)
+    for name, v in arrays.items():
+        if frac < 1.0:
+            rows = np.sort(np.random.RandomState(0).choice(len(v), int(len(v) * frac), replace=False))
+            v = v[rows]
+            np.save(os.path.join(path, name + '_rows.npy'), rows.astype(np.float64))
+        np.save(os.path.join(path, name + '.npy'), v)
 
 
 # ------------------------------------------------------------------------------------------------
@@ -110,11 +136,10 @@ class ClockSampler(threading.Thread):
 def load_weights(which):
     from tacotronv2_wavernn_chinese_b200 import synth
     if which in ('auto', 'shipped'):
-        for p in (CKPT_TRAVEL, CKPT_CONTAINER):
-            if os.path.isfile(p):
-                import torch
-                sd = torch.load(p, map_location='cpu', weights_only=True)
-                return {k: v.numpy() for k, v in sd.items()}, 'shipped checkpoint latest_weights.pyt (step 617k)'
+        if os.path.isfile(CKPT_TRAVEL):
+            import torch
+            sd = torch.load(CKPT_TRAVEL, map_location='cpu', weights_only=True)
+            return {k: v.numpy() for k, v in sd.items()}, 'shipped checkpoint latest_weights.pyt (step 617k)'
         if which == 'shipped':
             raise SystemExit('--weights shipped: no travel copy of the checkpoint (run __graft_entry__.build() in the container)')
     return synth.synth_state_dict(0), 'random-init weights of the shipped architecture (synth.synth_state_dict(0))'
@@ -312,13 +337,9 @@ def _taco_setup(local):
     from tacotronv2_wavernn_chinese_b200.tacotron.synthesizer import Synthesizer
     from tacotronv2_wavernn_chinese_b200.tacotron.text import Symbols
     npz = os.path.join(ROOT, 'oracle', '_ref', 'tacotron_weights.npz')
-    if os.path.isfile(npz):
-        w = dict(np.load(npz))
-    elif os.path.isdir('/root/reference/logs-Tacotron-2/taco_pretrained'):
-        from tacotronv2_wavernn_chinese_b200.tacotron import ckpt
-        w = ckpt.load_tacotron_weights('/root/reference/logs-Tacotron-2/taco_pretrained')
-    else:
-        raise SystemExit('no Tacotron checkpoint on this box (run __graft_entry__.build() in the container first)')
+    if not os.path.isfile(npz):
+        raise SystemExit(f'no Tacotron checkpoint: {npz} is made by __graft_entry__.build() from the reference checkout')
+    w = dict(np.load(npz))
     s = json.load(open(os.path.join(ROOT, 'tests', 'golden', 'taco_symbols.json'), encoding='utf-8'))
     syn = Synthesizer()
     syn.symbols = Symbols(s['symbols'])
@@ -362,6 +383,9 @@ def run_text2audio(args):
             dist.all_reduce(dt, op=dist.ReduceOp.MAX)
         if i >= args.warmup:
             times.append(float(dt.item()))
+    if rank == 0 and args.dump_outputs:
+        dump_outputs(args.dump_outputs, {'wave': np.concatenate(waves), 'wave_lengths': [len(w) for w in waves],
+                                         'mel': np.concatenate(mels), 'mel_frames': [len(m) for m in mels]})
     if rank == 0:
         total = int(sum(len(w) for w in waves))
         frames = [int(m.shape[0]) for m in mels]
@@ -416,6 +440,8 @@ def run_tacotron(args):
             times.append(time.perf_counter() - t0)
         nst = int(info['decode']['nsteps'][0])
     dt = float(np.mean(times))
+    if args.dump_outputs:
+        dump_outputs(args.dump_outputs, {'mel': mels[0]})
     # the decoder loop alone (CUDA events on the launch stream), encoder / postnet / host copies excluded
     ids = np.array([s['sentences']['241']['ids']], dtype=np.int32)
     mem = syn.engine.encode(ids, np.array([ids.shape[1]], dtype=np.int32))
@@ -515,7 +541,7 @@ def main():
         ev0, ev1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
         ev0.record()
         for i in range(steps):
-            one_step(i)
+            measure.last = one_step(i)
         ev1.record()
         sync_all()
         eng.check()
@@ -534,7 +560,7 @@ def main():
     sampler = ClockSampler(local)
     sampler.start()
     ms, gen_ms, launches = measure(B, rank * B, args.steps, args.warmup)
-    weak_kernel = measure.kernel
+    weak_kernel, weak_out = measure.kernel, measure.last
     clocks = sampler.stop()
     value = N * B * S * args.steps / (ms / 1e3)
 
@@ -632,6 +658,8 @@ def main():
         }
         if not args.no_cpu_baseline and N == 1:        # reported baseline: rank 0, single-GPU runs only
             line['cpu_baseline'] = cpu_baseline(B, T, 12.0)
+        if args.dump_outputs:                          # rank 0's utterances: labels [B, S], wave [B, (T - 1) * hop]
+            dump_outputs(args.dump_outputs, {'labels': weak_out['labels'], 'wave': weak_out['wave']})
         print(json.dumps(line), flush=True)
     if N > 1:
         dist.barrier()

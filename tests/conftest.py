@@ -10,7 +10,6 @@ if ROOT not in sys.path:
 
 def pytest_configure(config):
     config.addinivalue_line('markers', 'gpu: needs a real B200 (run with -m gpu on the GPU box)')
-    config.addinivalue_line('markers', 'reference: needs /root/reference (build container only)')
 
 
 @pytest.fixture(scope='session', autouse=True)
@@ -31,19 +30,17 @@ REF_CKPT_COPY = os.path.join(ROOT, 'oracle', '_ref', 'latest_weights.pyt')
 
 
 def load_ckpt_state_dict():
-    """The shipped checkpoint, from /root/reference (container) or the git-ignored travel copy oracle/_ref/."""
-    import numpy as np
+    """The shipped checkpoint, from the git-ignored copy that __graft_entry__.build() makes under oracle/_ref/, or None."""
     import torch
-    for p in ('/root/reference/logs_wavernn/checkpoints/latest_weights.pyt', REF_CKPT_COPY):
-        if os.path.isfile(p):
-            sd = torch.load(p, map_location='cpu', weights_only=False)
-            return {k: v.numpy() for k, v in sd.items()}
-    return None
+    if not os.path.isfile(REF_CKPT_COPY):
+        return None
+    sd = torch.load(REF_CKPT_COPY, map_location='cpu', weights_only=False)
+    return {k: v.numpy() for k, v in sd.items()}
 
 
 @pytest.fixture(scope='session')
 def ckpt_state_dict():
     sd = load_ckpt_state_dict()
     if sd is None:
-        pytest.skip('shipped checkpoint not available (neither /root/reference nor oracle/_ref/)')
+        pytest.skip('shipped checkpoint not available (no oracle/_ref/ copy)')
     return sd

@@ -6,7 +6,6 @@ import numpy as np
 
 from conftest import GOLDEN, ROOT
 
-REF_CKPT_DIR = '/root/reference/logs-Tacotron-2/taco_pretrained'
 TRAVEL_COPY = os.path.join(ROOT, 'oracle', '_ref', 'tacotron_weights.npz')
 
 SHAPES = {
@@ -46,9 +45,7 @@ def synth_taco_weights(seed=0):
 
 
 def real_taco_weights():
-    if os.path.isdir(REF_CKPT_DIR):
-        from tacotronv2_wavernn_chinese_b200.tacotron import ckpt
-        return ckpt.load_tacotron_weights(REF_CKPT_DIR)
+    """The shipped checkpoint's inference variables, from the copy __graft_entry__.build() makes under oracle/_ref/, or None."""
     if os.path.isfile(TRAVEL_COPY):
         return dict(np.load(TRAVEL_COPY))
     return None

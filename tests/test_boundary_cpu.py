@@ -2,6 +2,7 @@
 the hparams singleton / dsp / paths mirrors behave like the reference's, the CLI validates its input.
 No GPU compute is invoked here."""
 import ctypes
+import json
 import os
 import re
 import subprocess
@@ -88,17 +89,12 @@ print("OK")
     assert r.returncode == 0 and 'OK' in r.stdout, r.stdout + r.stderr
 
 
-@pytest.mark.reference
 def test_hparams_file_matches_reference_values():
-    ref = '/root/reference/wavernn_hparams.py'
-    if not os.path.isfile(ref):
-        pytest.skip('reference not present')
-    a, b = {}, {}
-    exec(open(ref).read(), a)
-    exec(open(os.path.join(ROOT, 'wavernn_hparams.py')).read(), b)
-    ka = {k: v for k, v in a.items() if not k.startswith('__')}
-    kb = {k: v for k, v in b.items() if not k.startswith('__')}
-    assert ka == kb
+    """Every value of wavernn_hparams.py equals the reference's (tests/golden/wavernn_hparams_from_reference.json,
+    oracle/make_golden_reference_files.py)."""
+    from oracle.make_golden_reference_files import hparams_values
+    ref = json.load(open(os.path.join(ROOT, 'tests', 'golden', 'wavernn_hparams_from_reference.json')))
+    assert hparams_values(os.path.join(ROOT, 'wavernn_hparams.py')) == ref
 
 
 def test_dsp_mirror_matches_oracle():
@@ -202,7 +198,7 @@ def test_bench_cpu_arm_helpers():
     bench._PORT[('t', 4)] = 2                                # skip the thread probe in the test
     pr = bench.port_sample(4, 0.3)
     assert pr['value'] > 0 and pr['steps'] >= 10 and pr['threads'] == 2
-    if bench.ref_model() is not None:                        # /root/reference or oracle/_ref/reference_src.zip
+    if bench.ref_model() is not None:                        # the reference's sources are present (oracle/_ref/reference_src.zip)
         import torch
         bench._REF[('threads', 4)] = 2
         r = bench.ref_sample(4, 0.3)
@@ -217,7 +213,7 @@ def test_reference_travel_copy_times_the_reference_loop():
     sample, and the memoised conditioning network returning what the reference module computed."""
     from oracle import ref_harness as rh
     if not rh.available():
-        pytest.skip('neither /root/reference nor the travel copy oracle/_ref/reference_src.zip is present')
+        pytest.skip('the reference sources are not present (oracle/_ref/reference_src.zip is made by __graft_entry__.build())')
     import torch
     m = rh.build_model()
     mel = torch.as_tensor(synth_mod.synth_mels(3, 2, 21))

@@ -19,7 +19,7 @@ def _run(args, cwd):
 
 
 def test_tacotron_synthesize_then_wavernn_gen(tmp_path):
-    wav_ckpt = REF_CKPT_COPY if os.path.isfile(REF_CKPT_COPY) else '/root/reference/logs_wavernn/checkpoints/latest_weights.pyt'
+    wav_ckpt = REF_CKPT_COPY
     if not (os.path.isfile(TRAVEL_COPY) and os.path.isfile(wav_ckpt)):
         pytest.skip('shipped checkpoints not available on this box')
     s = sentences()

@@ -5,22 +5,44 @@ import numpy as np
 import pytest
 
 from oracle import tacotron_oracle as to
-from taco_common import REF_CKPT_DIR, SHAPES, real_taco_weights, sentences, synth_taco_weights
+from conftest import GOLDEN
+from taco_common import SHAPES, real_taco_weights, sentences, synth_taco_weights
 
 
-def test_bundle_reader_shapes_and_step():
-    if not os.path.isdir(REF_CKPT_DIR):
-        pytest.skip('reference checkpoint directory not present')
+def _checkpoint_dir(d):
+    """The shipped checkpoint directory rebuilt from tests/golden/ (oracle/make_golden_reference_files.py): the real `checkpoint`
+    pointer file and .index, and a sparse stand-in for the 62 MB data shard that holds the sampled tensors' bytes where the
+    index places them (zeros elsewhere).  -> {name: raw bytes} of the sampled tensors."""
+    import shutil
+    prefix = d / 'tacotron_model.ckpt-206500'
+    shutil.copyfile(os.path.join(GOLDEN, 'taco_ckpt_checkpoint.txt'), d / 'checkpoint')
+    shutil.copyfile(os.path.join(GOLDEN, 'taco_ckpt.index'), str(prefix) + '.index')
+    z = np.load(os.path.join(GOLDEN, 'taco_ckpt_data_sample.npz'))
+    sampled = {}
+    with open(str(prefix) + '.data-00000-of-00001', 'wb') as f:
+        f.truncate(int(z['data_size']))
+        for i, name in enumerate(z['names']):
+            f.seek(int(z[f'offset_{i}']))
+            f.write(z[f'bytes_{i}'].tobytes())
+            sampled[str(name)] = z[f'bytes_{i}'].tobytes()
+    return sampled
+
+
+def test_bundle_reader_shapes_and_step(tmp_path):
     from tacotronv2_wavernn_chinese_b200.tacotron import ckpt
-    w = ckpt.load_tacotron_weights(REF_CKPT_DIR)          # resolves the TF `checkpoint` pointer file, skips Adam slots
+    sampled = _checkpoint_dir(tmp_path)
+    w = ckpt.load_tacotron_weights(str(tmp_path))          # resolves the TF `checkpoint` pointer file, skips Adam slots
     assert int(w['global_step']) == 206500
     for k, shp in SHAPES.items():
         assert w[k].shape == shp and w[k].dtype == np.float32, k
     assert not any(k.endswith('/Adam') or k.endswith('/Adam_1') for k in w)
     n = sum(v.size for k, v in w.items() if k != 'global_step')
     assert n == 5166370
-    idx = ckpt.read_index(ckpt.resolve_checkpoint(REF_CKPT_DIR) + '.index')
+    idx = ckpt.read_index(ckpt.resolve_checkpoint(str(tmp_path)) + '.index')
     assert idx['Tacotron_model/inference/inputs_embedding']['shape'] == (191, 128)
+    for name, raw in sampled.items():                      # the bytes come back from where the index says they are
+        key = name[len(ckpt.PREFIX):] if name.startswith(ckpt.PREFIX) else name
+        assert w[key].tobytes() == raw, name
 
 
 def test_symbol_table_pin():

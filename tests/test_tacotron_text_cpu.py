@@ -4,6 +4,7 @@ import os
 import numpy as np
 import pytest
 
+from conftest import GOLDEN
 from taco_common import sentences
 from tacotronv2_wavernn_chinese_b200.tacotron.text import Symbols, build_symbols
 
@@ -19,9 +20,8 @@ def test_symbols_roundtrip_and_eos():
 
 
 def test_build_symbols_matches_reference_scan(tmp_path):
-    ref = '/root/reference/train.txt'
-    if os.path.isfile(ref):
-        assert build_symbols(ref) == sentences()['symbols']
+    # the train.txt lines that introduce every symbol (oracle/make_golden_reference_files.py)
+    assert build_symbols(os.path.join(GOLDEN, 'train_symbol_lines.txt')) == sentences()['symbols']
     p = tmp_path / 't.txt'
     p.write_text('a|b|1|2|x|b a1 c\na|b|1|2|y|a1 d\n', encoding='utf-8')
     assert build_symbols(str(p)) == ['_', '~', 'a1', 'b', 'c', 'd']
