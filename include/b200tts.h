@@ -139,6 +139,19 @@ int b200tts_wavernn_upsample(b200tts_wavernn* ctx, const float* d_mel, int B, in
 int b200tts_wavernn_generate(b200tts_wavernn* ctx, const float* d_mel, int B, int T, const b200tts_rng* rng,
                              const b200tts_gen_opts* opts, int16_t* d_labels, double* d_wave, void* stream);
 
+/* STREAMING.  d_mel [B][feat][T] -> the same labels / wave as b200tts_wavernn_generate, and while the kernel runs, the final wave
+ * samples in h_wave [B][(T-1)*hop] (PINNED host memory the device can write, e.g. cudaHostAlloc / torch pin_memory); *h_progress =
+ * lock-steps whose samples are in h_wave (published every chunk_steps steps and at the end; < 0: the kernel gave up).  Sample n of
+ * every row is final once *h_progress > n.  The call stores 0 to *h_progress before it enqueues anything; both buffers must stay
+ * alive until the stream has passed the call.  Push kernel only: 1..32 rows, no folding, no packed rows, max_steps == 0, kernel
+ * auto or grid; everything else -> B200TTS_EINVAL (no counterpart in the reference, which returns audio only at the end). */
+int b200tts_wavernn_generate_stream(b200tts_wavernn* ctx, const float* d_mel, int B, int T, const b200tts_rng* rng,
+                                    const b200tts_gen_opts* opts, int chunk_steps, double* h_wave, int64_t* h_progress,
+                                    int16_t* d_labels, double* d_wave, void* stream);
+/* Host-only helper: acquire-loads *h_progress until it is >= at_least or < 0 or timeout_ms passes; returns B200TTS_OK and the
+ * last value seen in *progress (the caller decides what a timeout means).  Releases nothing, launches nothing, needs no device. */
+int b200tts_wavernn_stream_wait(const int64_t* h_progress, int64_t at_least, int timeout_ms, int64_t* progress);
+
 /* n_folds and fold_len = target + 2*overlap of fold_with_overlap (fatchord_version.py:319-330) for a T-frame utterance. */
 int b200tts_wavernn_fold_geometry(int T, int hop, int target, int overlap, int* n_folds, int* fold_len);
 

@@ -68,6 +68,9 @@ SIGNATURES = {
                                            C.c_void_p]),
     'b200tts_wavernn_generate': (C.c_int, [C.c_void_p, C.c_void_p, C.c_int, C.c_int, C.POINTER(Rng), C.POINTER(GenOpts),
                                            C.c_void_p, C.c_void_p, C.c_void_p]),
+    'b200tts_wavernn_generate_stream': (C.c_int, [C.c_void_p, C.c_void_p, C.c_int, C.c_int, C.POINTER(Rng), C.POINTER(GenOpts),
+                                                  C.c_int, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p]),
+    'b200tts_wavernn_stream_wait': (C.c_int, [C.c_void_p, C.c_int64, C.c_int, C.POINTER(C.c_int64)]),
     'b200tts_wavernn_fold_geometry': (C.c_int, [C.c_int, C.c_int, C.c_int, C.c_int, C.POINTER(C.c_int), C.POINTER(C.c_int)]),
     'b200tts_wavernn_generate_host': (C.c_int, [C.c_void_p, C.c_void_p, C.c_int, C.c_int, C.POINTER(Rng),
                                                 C.POINTER(GenOpts), C.c_void_p, C.c_void_p]),

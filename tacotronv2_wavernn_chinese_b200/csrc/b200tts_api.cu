@@ -3,12 +3,14 @@
 
 #include <cooperative_groups.h>
 #include <algorithm>
+#include <chrono>
 #include <cmath>
 #include <cstring>
 #include <cstdio>
 #include <cstdlib>
 #include <map>
 #include <string>
+#include <thread>
 #include <vector>
 
 #include "common.cuh"
@@ -821,12 +823,12 @@ static void launch_grid(b200tts_wavernn* ctx, const float* d_mel, GenArgs& ua, c
 }
 
 // ---- small-batch push kernel (wavernn_push.cuh) --------------------------------------------------------------------------
-template <int G>
+template <int G, bool STREAM>
 static void launch_push_t(b200tts_wavernn* ctx, PushArgs& a, cudaStream_t st) {
   const PushModel& pm = ctx->pm;
   using PT = PushTraits<G>;
   size_t smem = ((size_t)pm.blob + (size_t)PT::scratch_floats(a.hop, a.NT)) * sizeof(float);
-  auto kern = wavernn_push_kernel<G>;
+  auto kern = wavernn_push_kernel<G, STREAM>;
   B200_CUDA(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
   int per_sm = 0;
   B200_CUDA(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, kern, kPushThreads, smem));
@@ -861,8 +863,16 @@ struct PackInfo {            // gen_opts.d_pack_*: kernel rows run queues of utt
   const int* start;
   int rows, segs, steps, n_utt;
 };
+// b200tts_wavernn_generate_stream: the kernel also hands every final wave sample to pinned host memory (device aliases here)
+struct StreamWave {
+  double* h_wave;
+  long long* h_progress;
+  int chunk_steps;
+  const int* utt_frames;
+  int fade_len, mu_law;
+};
 static void launch_push(b200tts_wavernn* ctx, const float* d_mel, GenArgs& ua, cudaStream_t st, const FoldGeom* fold, int T0,
-                        const PackInfo* pack = nullptr) {
+                        const PackInfo* pack = nullptr, const StreamWave* sw = nullptr) {
   const b200tts_wavernn_cfg& c = ctx->cfg;
   const PushModel& pm = ctx->pm;
   const int rows = pack ? pack->rows : ua.B;
@@ -903,6 +913,11 @@ static void launch_push(b200tts_wavernn* ctx, const float* d_mel, GenArgs& ua, c
   a.S_src = T * hop;
   a.rng_mode = ua.rng_mode; a.seed = ua.seed; a.utt_offset = ua.utt_offset; a.utt_ids = ua.utt_ids; a.q = ua.q;
   a.teacher = ua.teacher; a.logits_out = ua.logits_out; a.labels = ua.labels;
+  if (sw) {
+    REQUIRE(ng == 1 && !fold && !pack, B200TTS_EINVAL, "internal: streaming needs a plain batch of <= 32 rows");
+    a.h_wave = sw->h_wave; a.h_progress = sw->h_progress; a.chunk_steps = sw->chunk_steps;
+    a.d_utt_frames = sw->utt_frames; a.fade_len = sw->fade_len; a.mu_law = sw->mu_law;
+  }
   a.prof = nullptr;
   if (getenv("B200TTS_GRID_PROF")) {
     ctx->push_prof.ensure((size_t)pm.ncta * 12 * sizeof(long long));
@@ -924,11 +939,16 @@ static void launch_push(b200tts_wavernn* ctx, const float* d_mel, GenArgs& ua, c
     void* args[] = {(void*)&m, (void*)&a};
     B200_CUDA(cudaLaunchCooperativeKernel((const void*)wavernn_pushmg_kernel, dim3(pm.ncta), dim3(kPushThreads), args, smem, st));
     ctx->launches++;
+  } else if (sw) switch (G) {
+    case 4: launch_push_t<4, true>(ctx, a, st); break;
+    case 8: launch_push_t<8, true>(ctx, a, st); break;
+    case 16: launch_push_t<16, true>(ctx, a, st); break;
+    default: launch_push_t<32, true>(ctx, a, st); break;
   } else switch (G) {
-    case 4: launch_push_t<4>(ctx, a, st); break;
-    case 8: launch_push_t<8>(ctx, a, st); break;
-    case 16: launch_push_t<16>(ctx, a, st); break;
-    default: launch_push_t<32>(ctx, a, st); break;
+    case 4: launch_push_t<4, false>(ctx, a, st); break;
+    case 8: launch_push_t<8, false>(ctx, a, st); break;
+    case 16: launch_push_t<16, false>(ctx, a, st); break;
+    default: launch_push_t<32, false>(ctx, a, st); break;
   }
   B200_CUDA(cudaEventRecord(ctx->ev1, st));
 }
@@ -1043,7 +1063,8 @@ static void check_grid_error(b200tts_wavernn* ctx) {
 }
 
 static void run_generate_rows(b200tts_wavernn* ctx, const float* d_mel, int B, int T, const b200tts_rng* rng,
-                              const b200tts_gen_opts* opts, int16_t* d_labels, double* d_wave, cudaStream_t st);
+                              const b200tts_gen_opts* opts, int16_t* d_labels, double* d_wave, cudaStream_t st,
+                              StreamWave* sw = nullptr);
 
 // The wide mapping streams a sample-rate mel buffer [S][feat][Bp] (1.8 GB at 256 rows x 80 frames, 22.5 GB at 256 x 1000): long
 // utterances x large batches would run out of memory before anything else.  Such a call is cut into row ranges whose buffers stay
@@ -1088,7 +1109,8 @@ static void run_generate(b200tts_wavernn* ctx, const float* d_mel, int B, int T,
 }
 
 static void run_generate_rows(b200tts_wavernn* ctx, const float* d_mel, int B, int T, const b200tts_rng* rng,
-                              const b200tts_gen_opts* opts, int16_t* d_labels, double* d_wave, cudaStream_t st) {
+                              const b200tts_gen_opts* opts, int16_t* d_labels, double* d_wave, cudaStream_t st,
+                              StreamWave* sw) {
   const b200tts_wavernn_cfg& c = ctx->cfg;
   const int hop = c.hop_length, S = T * hop, O = c.res_out_dims;
   b200tts_gen_opts o{};
@@ -1102,7 +1124,7 @@ static void run_generate_rows(b200tts_wavernn* ctx, const float* d_mel, int B, i
   const int steps = o.max_steps ? o.max_steps : S;
   const int fade_len = 20 * hop;                      // fatchord_version.py:256
   const int wave_len = (T - 1) * hop;                 // :184
-  if (d_wave) {
+  if (d_wave || sw) {
     REQUIRE(steps == S, B200TTS_EINVAL, "a wave needs all steps (max_steps must be 0)");
     REQUIRE(wave_len >= fade_len, B200TTS_EINVAL,
             "T must be >= 21 frames: the reference's 20-hop fade-out (fatchord_version.py:256-258) fails below that");
@@ -1159,6 +1181,8 @@ static void run_generate_rows(b200tts_wavernn* ctx, const float* d_mel, int B, i
   }
   const bool use_push = !use_tc && kernel == B200TTS_KERNEL_GRID && push_eligible(ctx, packing ? o.pack_rows : GB);
   REQUIRE(!packing || use_push, B200TTS_EINVAL, "packed generation needs the push kernel (kernel=auto/grid, rnn_dims = fc_dims = 512)");
+  REQUIRE(!sw || (use_push && GB <= kMgG), B200TTS_EINVAL,
+          "streaming needs the push kernel (kernel=auto/grid, 1..32 rows, rnn_dims = fc_dims = 512)");
   if (kernel == B200TTS_KERNEL_GRID && !ctx->gm.ok)
     throw Error(B200TTS_EINVAL, "kernel=grid was requested but this model/device cannot run the weight-stationary grid kernel "
                                 "(needs rnn_dims == fc_dims, n_classes == 2*rnn_dims, cooperative launch, R/4 <= SM count)");
@@ -1205,7 +1229,8 @@ static void run_generate_rows(b200tts_wavernn* ctx, const float* d_mel, int B, i
     launch_tc(ctx, d_mel, a, st);
   } else if (use_push) {
     PackInfo pi{o.d_pack_utt, o.d_pack_start, o.pack_rows, o.pack_segs, o.pack_steps, B};
-    launch_push(ctx, d_mel, a, st, folding ? &fg : nullptr, T, packing ? &pi : nullptr);
+    if (sw) { sw->utt_frames = o.d_utt_frames; sw->fade_len = fade_len; sw->mu_law = o.mu_law; }
+    launch_push(ctx, d_mel, a, st, folding ? &fg : nullptr, T, packing ? &pi : nullptr, sw);
   } else {
     launch_grid(ctx, d_mel, a, st, folding ? &fg : nullptr, S);
   }
@@ -1241,6 +1266,71 @@ extern "C" int b200tts_wavernn_generate(b200tts_wavernn* ctx, const float* d_mel
   REQUIRE(B >= 1 && T >= 1 && B <= 65535, B200TTS_EINVAL, "B must be 1..65535 and T positive");
   DeviceGuard dg(ctx->device);
   run_generate(ctx, d_mel, B, T, rng, opts, d_labels, d_wave, (cudaStream_t)stream);
+  API_END
+}
+
+// Pinned host memory the device can write: the device alias of [p, p + bytes).  Pageable memory cannot be written by a running
+// kernel (it would need a copy, i.e. the end of the kernel) -> EINVAL.
+static void* host_alias(void* p, size_t bytes, const char* name) {
+  for (const char* q : {(const char*)p, (const char*)p + bytes - 1}) {
+    cudaPointerAttributes at{};
+    B200_CUDA(cudaPointerGetAttributes(&at, q));
+    REQUIRE(at.type == cudaMemoryTypeHost, B200TTS_EINVAL,
+            std::string(name) + " must be PINNED host memory the device can write (cudaHostAlloc / torch pin_memory), not pageable "
+            "or device memory");
+  }
+  void* d = nullptr;
+  const cudaError_t e = cudaHostGetDevicePointer(&d, p, 0);
+  if (e != cudaSuccess) {
+    cudaGetLastError();
+    throw Error(B200TTS_EINVAL, std::string(name) + ": pinned memory not mapped into the device address space: " + cudaGetErrorString(e));
+  }
+  return d;
+}
+
+extern "C" int b200tts_wavernn_generate_stream(b200tts_wavernn* ctx, const float* d_mel, int B, int T, const b200tts_rng* rng,
+                                               const b200tts_gen_opts* opts, int chunk_steps, double* h_wave, int64_t* h_progress,
+                                               int16_t* d_labels, double* d_wave, void* stream) {
+  API_BEGIN
+  REQUIRE(ctx && d_mel && h_wave && h_progress, B200TTS_EINVAL, "null argument");
+  REQUIRE(chunk_steps >= 1, B200TTS_EINVAL, "chunk_steps must be >= 1");
+  REQUIRE(B >= 1 && B <= 32 && T >= 1, B200TTS_EINVAL, "streaming takes 1..32 rows (the push kernel) and T positive");
+  REQUIRE(((uintptr_t)h_progress & 7) == 0, B200TTS_EINVAL, "h_progress must be 8-byte aligned");
+  if (opts) {
+    REQUIRE(opts->fold_target == 0, B200TTS_EINVAL, "streaming does not take fold-with-overlap generation (its output crosses folds)");
+    REQUIRE(!opts->d_pack_utt, B200TTS_EINVAL, "streaming does not take packed rows (an utterance would start mid-launch)");
+    REQUIRE(opts->max_steps == 0, B200TTS_EINVAL, "streaming produces the whole wave (max_steps must be 0)");
+    REQUIRE(opts->kernel == B200TTS_KERNEL_AUTO || opts->kernel == B200TTS_KERNEL_GRID, B200TTS_EINVAL,
+            "streaming runs the push kernel only (kernel=auto or grid)");
+  }
+  REQUIRE(T >= 21, B200TTS_EINVAL, "T must be >= 21 frames: the reference's 20-hop fade-out (fatchord_version.py:256-258) fails below that");
+  // the kernel choice (push kernel only) is made by run_generate_rows, like for b200tts_wavernn_generate
+  void* dp = host_alias(h_progress, sizeof(int64_t), "h_progress");        // first CUDA call: ECUDA without a device
+  DeviceGuard dg(ctx->device);
+  const size_t wl = (size_t)(T - 1) * ctx->cfg.hop_length;
+  void* dw = host_alias(h_wave, (size_t)B * wl * sizeof(double), "h_wave");
+  __atomic_store_n(h_progress, (int64_t)0, __ATOMIC_RELEASE);
+  StreamWave sw{reinterpret_cast<double*>(dw), reinterpret_cast<long long*>(dp), chunk_steps, nullptr, 0, 0};
+  run_generate_rows(ctx, d_mel, B, T, rng, opts, d_labels, d_wave, (cudaStream_t)stream, &sw);
+  API_END
+}
+
+extern "C" int b200tts_wavernn_stream_wait(const int64_t* h_progress, int64_t at_least, int timeout_ms, int64_t* progress) {
+  API_BEGIN
+  REQUIRE(h_progress && progress, B200TTS_EINVAL, "null argument");
+  REQUIRE(timeout_ms >= 0, B200TTS_EINVAL, "timeout_ms must be >= 0");
+  const auto t0 = std::chrono::steady_clock::now();
+  const auto limit = t0 + std::chrono::milliseconds(timeout_ms);
+  int64_t v = __atomic_load_n(h_progress, __ATOMIC_ACQUIRE);
+  // spin for the first 200 us (a chunk of 275 steps takes 2.5-5.6 ms, the first one is what time-to-audio measures), then sleep
+  // in 50-us naps: a waiting thread costs no core while the kernel runs for seconds
+  for (unsigned it = 0; v < at_least && v >= 0; ++it) {
+    const auto now = std::chrono::steady_clock::now();
+    if (now >= limit) break;
+    if (now - t0 > std::chrono::microseconds(200)) std::this_thread::sleep_for(std::chrono::microseconds(50));
+    v = __atomic_load_n(h_progress, __ATOMIC_ACQUIRE);
+  }
+  *progress = v;
   API_END
 }
 

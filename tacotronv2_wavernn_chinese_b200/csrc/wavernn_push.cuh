@@ -84,6 +84,15 @@ struct PushArgs {
   const int* pack_utt;           // [pack_rows][pack_segs]
   const int* pack_start;         // [pack_rows][pack_segs + 1]
   int pack_segs, pack_rows;      // kernel rows >= pack_rows are idle
+  // STREAMING (wavernn_push_kernel<G, true>, b200tts_wavernn_generate_stream; plain batches only): while it runs, CTA 0 writes
+  // the final fp64 wave sample of every row -- the value finish_wave_kernel writes for the same label and position -- to
+  // caller-owned pinned host memory and publishes how many lock-steps are there.  Appended last: the offsets of the fields
+  // above, and with them the code of every other kernel that takes PushArgs, stay as they are.
+  double* h_wave;                // device alias of pinned host memory [B][(T-1)*hop]
+  long long* h_progress;         // device alias of a pinned int64: lock-steps whose samples are in h_wave (< 0: the kernel gave up)
+  int chunk_steps;               // publish every chunk_steps lock-steps (and once after the last)
+  const int* d_utt_frames;       // optional [B]: own frame count of each row (truncation / fade as finish_wave_kernel)
+  int fade_len, mu_law;
 };
 
 struct PushRowState {            // per-row bookkeeping in shared memory (normal mode: row u == utterance u from step 0, forever)
@@ -344,7 +353,37 @@ __device__ __forceinline__ void push_cond20(const PushArgs& A, const PushRowStat
   }
 }
 
+// ---- streaming (STREAM = true) ----------------------------------------------------------------------------------------
+// The samples are written and published by the LAST G threads of CTA 0 -- never gate threads (tid < 4G <= 128), which run the
+// gpu-scope fence of the re-arm every step and would otherwise wait there for host-bound stores -- in the shadow of the fc2
+// exchange.  Sample n of a row is final once the winner of step n is known (P01 of step n+1); it is stored in step n+1's P4
+// shadow, so after the P4 barrier of step t the samples of steps < t-1 are in h_wave: t-1 is what step t may publish.
+struct PushStreamSmem {
+  double dec[1024];              // wave_decode of every label (the fp64 pow of decode_mu_law leaves the per-step path)
+  double step;                   // wave_fade_step(fade_len)
+  int wlen[32];                  // own wave length of every row
+  int lab[32];                   // label of the step collected in this step's P01 (written by the gate threads)
+};
+__device__ __forceinline__ PushStreamSmem& push_stream_smem() {
+  __shared__ PushStreamSmem s;   // allocated only in the kernels that call this: the streaming instantiations
+  return s;
+}
+__device__ __forceinline__ void push_stream_publish(const PushArgs& A, long long steps_done) {
+  // the block barrier before this call orders CTA 0's earlier sample stores; the fence makes them visible system-wide
+  // before the count that announces them (the host reads it with an acquire load)
+  asm volatile("fence.acq_rel.sys;" ::: "memory");
+  asm volatile("st.release.sys.global.s64 [%0], %1;" ::"l"(A.h_progress), "l"(steps_done) : "memory");
+}
 template <int G>
+__device__ __forceinline__ void push_stream_sample(const PushArgs& A, const PushStreamSmem& ss, int tid, int n) {
+  const int u = tid - (kPushThreads - G);
+  const int wave_len_max = (A.T - 1) * A.hop;
+  if (u < 0 || u >= A.B || n >= wave_len_max) return;      // (the last hop of steps is not part of the wave, :184)
+  const int wl = ss.wlen[u];
+  A.h_wave[(size_t)u * wave_len_max + n] = n < wl ? wave_fade(ss.dec[ss.lab[u]], n, wl, A.fade_len, ss.step) : 0.0;
+}
+
+template <int G, bool STREAM>
 __global__ void __launch_bounds__(kPushThreads, 1) wavernn_push_kernel(PushModel M, PushArgs A) {
   using PT = PushTraits<G>;
   constexpr int NU = PT::NU;
@@ -406,6 +445,14 @@ __global__ void __launch_bounds__(kPushThreads, 1) wavernn_push_kernel(PushModel
     R.t0[tid] = 0;
     R.end[tid] = live ? A.pack_start[tid * (A.pack_segs + 1) + 1] : 0x7fffffff;
   }
+  if constexpr (STREAM) {
+    if (c == 0) {
+      PushStreamSmem& ss = push_stream_smem();
+      for (int l = tid; l < M.NC; l += kPushThreads) ss.dec[l] = wave_decode(l, (double)(M.NC - 1), A.mu_law);
+      if (tid < A.B && tid < G) ss.wlen[tid] = wave_row_len(A.d_utt_frames, tid, (A.T - 1) * A.hop, A.hop);
+      if (tid == 0) ss.step = wave_fade_step(A.fade_len);
+    }
+  }
   __syncthreads();
 
   PollGuard pg{A.error, 0, 0, false};
@@ -423,6 +470,14 @@ __global__ void __launch_bounds__(kPushThreads, 1) wavernn_push_kernel(PushModel
       s_pf[slot] += now_ - s_tmark;              \
       s_tmark = now_;                            \
     }                                            \
+  } while (0)
+  // a poll gave up (~2 s without a peer): the whole block leaves; a streaming CTA 0 first tells the host waiters
+#define PUSH_GIVE_UP()                                                                 \
+  do {                                                                                 \
+    if constexpr (STREAM) {                                                            \
+      if (c == 0 && tid == kPushThreads - 1) push_stream_publish(A, -1);               \
+    }                                                                                  \
+    return;                                                                            \
   } while (0)
 
   constexpr int NCQ = kPushThreads / G, NREC = 128 / NCQ;   // winner records per thread = G/4
@@ -457,7 +512,7 @@ __global__ void __launch_bounds__(kPushThreads, 1) wavernn_push_kernel(PushModel
         bestp = other > bestp ? other : bestp;
       }
       if (lane < G) smax[warp * G + lane] = bestp;
-      if (__syncthreads_or(pg.aborted ? 1 : 0)) return;
+      if (__syncthreads_or(pg.aborted ? 1 : 0)) PUSH_GIVE_UP();
       if (gate) {                                           // every warp covered different producers: reduce the 16 warps
         unsigned long long b = 0ull;
 #pragma unroll
@@ -465,7 +520,10 @@ __global__ void __launch_bounds__(kPushThreads, 1) wavernn_push_kernel(PushModel
         const int label = (int)push_cls(b);
         const int putt = R.putt[gu], pn = R.pn[gu];         // where this row was at step t-1
         if (putt >= 0) {
-          if (c == 0 && gj == 0) A.labels[(size_t)putt * A.S + pn] = (int16_t)label;
+          if (c == 0 && gj == 0) {
+            A.labels[(size_t)putt * A.S + pn] = (int16_t)label;
+            if constexpr (STREAM) push_stream_smem().lab[gu] = label;
+          }
           const int fb = A.teacher ? (int)A.teacher[(size_t)putt * A.S + pn] : label;
           x = label_to_float(fb, ncls_m1);
         }
@@ -508,7 +566,7 @@ __global__ void __launch_bounds__(kPushThreads, 1) wavernn_push_kernel(PushModel
       push_mma<G, 16>(Wb + M.oih2, a, partX, ul, kq, warp, lane);
     }
     PUSH_MARK(2);
-    if (__syncthreads_or(pg.aborted ? 1 : 0)) return;
+    if (__syncthreads_or(pg.aborted ? 1 : 0)) PUSH_GIVE_UP();
     if (gate) {
       const float* cd = cond20;
       const float* bhh = Wb + M.obhh2;
@@ -528,7 +586,7 @@ __global__ void __launch_bounds__(kPushThreads, 1) wavernn_push_kernel(PushModel
     // shadow: W_hh1 . h1(t) for step t+1
     if constexpr (kPrefetchH1) push_mma<G, 12>(Wb + M.ohh1, reinterpret_cast<const float4 (&)[PT::NL]>(ah1), partY, ul, kq, warp, lane);
     else push_gemm<G, 12>(Wb + M.ohh1, vecp(PV_H1, par), partY, ul, kq, warp, lane, pg);
-    if (__syncthreads_or(pg.aborted ? 1 : 0)) return;
+    if (__syncthreads_or(pg.aborted ? 1 : 0)) PUSH_GIVE_UP();
     for (int i = tid; i < 12 * G; i += kPushThreads) gh1[i] = push_part_sum<G, 12>(partY, i / G, i % G);
     PUSH_MARK(4);
 
@@ -538,7 +596,7 @@ __global__ void __launch_bounds__(kPushThreads, 1) wavernn_push_kernel(PushModel
       push_load<G>(vecp(PV_H2, par), a, ul, kq, pg);
       push_mma<G, 4>(Wb + M.ofc1, a, partX, ul, kq, warp, lane);
       PUSH_MARK(5);
-      if (__syncthreads_or(pg.aborted ? 1 : 0)) return;
+      if (__syncthreads_or(pg.aborted ? 1 : 0)) PUSH_GIVE_UP();
       if (gate) {
         const float v = (f1x + push_part_sum<G, 4>(partX, gj, gu)) + cond20[(12 + gj) * G + gu];
         st_relaxed_f32(vecp(PV_F1, par) + ((size_t)c * G + gu) * 4 + gj, fmaxf(v, 0.f));
@@ -546,7 +604,7 @@ __global__ void __launch_bounds__(kPushThreads, 1) wavernn_push_kernel(PushModel
       __syncwarp();
       push_mma<G, 12>(Wb + M.ohh2, a, partY, ul, kq, warp, lane);
     }
-    if (__syncthreads_or(pg.aborted ? 1 : 0)) return;
+    if (__syncthreads_or(pg.aborted ? 1 : 0)) PUSH_GIVE_UP();
     for (int i = tid; i < 12 * G; i += kPushThreads) gh2[i] = push_part_sum<G, 12>(partY, i / G, i % G);
     PUSH_MARK(6);
 
@@ -555,7 +613,7 @@ __global__ void __launch_bounds__(kPushThreads, 1) wavernn_push_kernel(PushModel
     // the fc2 conditioning value is taken BEFORE the barrier: after it the other threads may refresh cond20 for the next frame
     const float cv4 = gate ? cond20[(16 + gj) * G + gu] : 0.f;
     PUSH_MARK(7);
-    if (__syncthreads_or(pg.aborted ? 1 : 0)) return;
+    if (__syncthreads_or(pg.aborted ? 1 : 0)) PUSH_GIVE_UP();
     if (gate) {
       const float v = push_part_sum<G, 4>(partX, gj, gu) + cv4;
       const size_t e = ((size_t)c * G + gu) * 4 + gj;
@@ -571,6 +629,12 @@ __global__ void __launch_bounds__(kPushThreads, 1) wavernn_push_kernel(PushModel
       asm volatile("fence.acq_rel.gpu;" ::: "memory");
     }
     __syncwarp();
+    if constexpr (STREAM) {      // shadow: sample of step t-1 to the host; every chunk_steps steps announce the samples of steps < t-1
+      if (c == 0 && t > 0) {
+        push_stream_sample<G>(A, push_stream_smem(), tid, t - 1);
+        if (tid == kPushThreads - 1 && t > 1 && (t - 1) % A.chunk_steps == 0) push_stream_publish(A, t - 1);
+      }
+    }
     // shadow: conditioning of step t+1 (rows 0-15 into the other parity buffer; rows 16-35 only when a new frame starts)
     if (t + 1 < A.steps) {
       push_cond16<G>(A, R, fir_s, cond16 + (par ^ 1) * 16 * G, c, ncta, t + 1, tid);
@@ -581,7 +645,7 @@ __global__ void __launch_bounds__(kPushThreads, 1) wavernn_push_kernel(PushModel
     // ================= P5: fc3 on f2(t) + Gumbel-max over this CTA's 8 classes =================
     push_gemm<G, 8>(Wb + M.ofc3, vecp(PV_F2, par), partY, ul, kq, warp, lane, pg);
     PUSH_MARK(9);
-    if (__syncthreads_or(pg.aborted ? 1 : 0)) return;
+    if (__syncthreads_or(pg.aborted ? 1 : 0)) PUSH_GIVE_UP();
     if (tid < 8 * G) {
       const int r = tid / G, u = tid % G;
       const int cls = c * kCPC + r;
@@ -624,8 +688,17 @@ __global__ void __launch_bounds__(kPushThreads, 1) wavernn_push_kernel(PushModel
     __syncwarp();
     PUSH_MARK(10);
   }
+  if constexpr (STREAM) {        // the last trip collected the winner of step steps-1 and left before its P4: store, then announce all
+    if (c == 0) {
+      __syncthreads();
+      if (A.steps > 0) push_stream_sample<G>(A, push_stream_smem(), tid, A.steps - 1);
+      __syncthreads();
+      if (tid == kPushThreads - 1) push_stream_publish(A, A.steps);
+    }
+  }
   if (A.prof && tid == 0)
     for (int i = 0; i < 12; ++i) A.prof[(size_t)c * 12 + i] = s_pf[i];
+#undef PUSH_GIVE_UP
 #undef PUSH_MARK
 }
 

@@ -218,6 +218,32 @@ __global__ void xfade_unfold_kernel(const int16_t* __restrict__ labels /*[nfold]
   }
 }
 
+// The two halves of the generate() epilogue for ONE sample, shared by finish_wave_kernel and the streaming push kernel (which
+// decodes through a table built with wave_decode and fades in the loop), so that both produce the same bits:
+//   wave_decode: label -> float64, decode_mu_law (dsp.py:98-103) when mu_law is set
+//   wave_fade:   20-hop linear fade-out of sample i of a row truncated at wave_len (fatchord_version.py:256-258);
+//                step = wave_fade_step(fade_len) = np.linspace(1, 0, fade_len)[1]
+__device__ __forceinline__ double wave_decode(int label, double mu, int mu_law) {
+  float yf = label_to_float(label, (float)mu);
+  double y = (double)yf;
+  if (mu_law) {
+    double a = fabs(y);
+    double sgn = (y > 0.0) - (y < 0.0);
+    y = sgn / mu * (pow(1.0 + mu, a) - 1.0);
+  }
+  return y;
+}
+__device__ __forceinline__ double wave_fade_step(int fade_len) { return -1.0 / (double)(fade_len - 1); }
+__device__ __forceinline__ double wave_fade(double y, int i, int wave_len, int fade_len, double step) {
+  int k = i - (wave_len - fade_len);
+  if (k >= 0) y *= (k == fade_len - 1) ? 0.0 : (1.0 + (double)k * step);
+  return y;
+}
+// length of row b of a ragged batch: its own (T_b - 1) * hop, capped at the launch's
+__device__ __forceinline__ int wave_row_len(const int* utt_frames, int b, int wave_len_max, int hop) {
+  return utt_frames ? min(wave_len_max, max(0, (utt_frames[b] - 1) * hop)) : wave_len_max;
+}
+
 // generate() epilogue (fatchord_version.py:243-258): float64, decode_mu_law (dsp.py:98-103), truncate, 20-hop fade.
 // `utt_frames` (optional, [B]): true frame count of each row of a zero-padded ragged batch -> that row is truncated / faded at
 // ITS OWN (T_b - 1) * hop like a batch-1 run of the reference, and zero beyond.
@@ -227,19 +253,11 @@ __global__ void finish_wave_kernel(const int16_t* __restrict__ labels /*[B][S]*/
   const int b = blockIdx.y;
   const bool poisoned = gen_error && *gen_error;    // the generation kernel timed out: never hand back plausible-looking audio
   const double mu = (double)(ncls - 1);
-  const double step = -1.0 / (double)(fade_len - 1);   // np.linspace(1, 0, fade_len)
-  const int wave_len = utt_frames ? min(wave_len_max, max(0, (utt_frames[b] - 1) * hop)) : wave_len_max;
+  const double step = wave_fade_step(fade_len);
+  const int wave_len = wave_row_len(utt_frames, b, wave_len_max, hop);
   for (int i = blockIdx.x * blockDim.x + threadIdx.x; i < wave_len_max; i += gridDim.x * blockDim.x) {
     if (i >= wave_len) { wave[(size_t)b * wave_len_max + i] = 0.0; continue; }
-    float yf = label_to_float((int)labels[(size_t)b * S + i], (float)(ncls - 1));
-    double y = (double)yf;
-    if (mu_law) {
-      double a = fabs(y);
-      double sgn = (y > 0.0) - (y < 0.0);
-      y = sgn / mu * (pow(1.0 + mu, a) - 1.0);
-    }
-    int k = i - (wave_len - fade_len);
-    if (k >= 0) y *= (k == fade_len - 1) ? 0.0 : (1.0 + (double)k * step);
+    const double y = wave_fade(wave_decode((int)labels[(size_t)b * S + i], mu, mu_law), i, wave_len, fade_len, step);
     wave[(size_t)b * wave_len_max + i] = poisoned ? nan("") : y;
   }
 }

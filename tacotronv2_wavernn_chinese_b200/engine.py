@@ -122,62 +122,129 @@ class WaveRNNEngine:
             wave = None
             if want_wave and steps == GS:
                 wave = torch.empty(B, (T - 1) * self.hop, device=dev, dtype=torch.float64)
-            rng = Rng()
-            rng.seed = int(seed) & 0xFFFFFFFFFFFFFFFF
-            rng.utterance_offset = int(utterance_offset)
-            ids = None
-            if utterance_ids is not None:       # rows that are NOT consecutive utterances (length-sorted chunks): per-row global index
-                ids = torch.as_tensor(np.asarray(utterance_ids, dtype=np.int64)).to(dev).contiguous()
-                if tuple(ids.shape) != (B,) or fold is not None:
-                    raise ValueError('utterance_ids must be [B] (and cannot be combined with fold)')
-                rng.d_utterance_ids = ids.data_ptr()
-            qd = None
-            if q is not None:
-                qd = torch.as_tensor(q).to(device=dev, dtype=torch.float32).contiguous()
-                if qd.dim() != 3 or tuple(qd.shape[1:]) != (GB, self.n_classes) or qd.shape[0] < steps:
-                    raise ValueError(f'q must be [>= {steps}, {GB}, {self.n_classes}], got {tuple(qd.shape)}')
-                rng.mode = _lib.RNG_EXT_EXPONENTIAL
-                rng.d_q = qd.data_ptr()
-            else:
-                rng.mode = _lib.RNG_PHILOX
-            opts = GenOpts()
-            opts.kernel = _lib.KERNELS[kernel]
-            opts.mu_law = 1 if mu_law else 0
-            opts.max_steps = int(max_steps)
-            if fold is not None:
-                opts.fold_target, opts.fold_overlap = int(fold[0]), int(fold[1])
-            pk_u = pk_s = None
-            if pack is not None:
-                pk_u = torch.as_tensor(np.ascontiguousarray(pack['utt'], dtype=np.int32)).to(dev)
-                pk_s = torch.as_tensor(np.ascontiguousarray(pack['start'], dtype=np.int32)).to(dev)
-                rows, segs = pk_u.shape
-                if tuple(pk_s.shape) != (rows, segs + 1) or rows != int(pack['rows']):
-                    raise ValueError('pack: utt must be [rows, segs], start [rows, segs + 1]')
-                opts.d_pack_utt, opts.d_pack_start = pk_u.data_ptr(), pk_s.data_ptr()
-                opts.pack_rows, opts.pack_segs, opts.pack_steps = rows, segs, int(pack['steps'])
-            uf = None
-            if utt_frames is not None:
-                uf = torch.as_tensor(utt_frames).to(device=dev, dtype=torch.int32).contiguous()
-                if tuple(uf.shape) != (B,):
-                    raise ValueError('utt_frames must be [B]')
-                opts.d_utt_frames = uf.data_ptr()
-            td = None
-            if teacher is not None:
-                td = torch.as_tensor(teacher).to(device=dev, dtype=torch.int16).contiguous()
-                if tuple(td.shape) != (GB, GS):
-                    raise ValueError('teacher must be [B, S] ([n_folds, fold_len] when folding)')
-                opts.d_teacher = td.data_ptr()
-            logits = None
-            if return_logits:
-                logits = torch.empty(steps, GB, self.n_classes, device=dev, dtype=torch.float32)
-                opts.d_logits = logits.data_ptr()
+            rng, opts, keep, logits = self._call_args(B, GB, GS, steps, seed=seed, utterance_offset=utterance_offset,
+                                                      utterance_ids=utterance_ids, q=q, teacher=teacher, return_logits=return_logits,
+                                                      mu_law=mu_law, kernel=kernel, max_steps=max_steps, fold=fold,
+                                                      utt_frames=utt_frames, pack=pack)
             _lib.check(self.lib.b200tts_wavernn_generate(self._h, _ptr(m), B, T, C.byref(rng), C.byref(opts),
                                                          _ptr(labels), _ptr(wave), self._stream()))
             # keep inputs alive until the stream has consumed them
-            for t in (m, qd, td, uf, ids, pk_u, pk_s):
-                if t is not None:
-                    t.record_stream(torch.cuda.current_stream(self.device))
+            for t in [m] + keep:
+                t.record_stream(torch.cuda.current_stream(self.device))
         return dict(labels=labels, wave=wave, logits=logits, steps=steps)
+
+    def _call_args(self, B, GB, GS, steps, *, seed, utterance_offset, utterance_ids, q, teacher, return_logits, mu_law, kernel,
+                   max_steps, fold, utt_frames, pack):
+        """Rng / GenOpts of a generate call, the device tensors they point to, and the logits buffer (or None)."""
+        dev = self._dev()
+        rng = Rng()
+        rng.seed = int(seed) & 0xFFFFFFFFFFFFFFFF
+        rng.utterance_offset = int(utterance_offset)
+        ids = None
+        if utterance_ids is not None:       # rows that are NOT consecutive utterances (length-sorted chunks): per-row global index
+            ids = torch.as_tensor(np.asarray(utterance_ids, dtype=np.int64)).to(dev).contiguous()
+            if tuple(ids.shape) != (B,) or fold is not None:
+                raise ValueError('utterance_ids must be [B] (and cannot be combined with fold)')
+            rng.d_utterance_ids = ids.data_ptr()
+        qd = None
+        if q is not None:
+            qd = torch.as_tensor(q).to(device=dev, dtype=torch.float32).contiguous()
+            if qd.dim() != 3 or tuple(qd.shape[1:]) != (GB, self.n_classes) or qd.shape[0] < steps:
+                raise ValueError(f'q must be [>= {steps}, {GB}, {self.n_classes}], got {tuple(qd.shape)}')
+            rng.mode = _lib.RNG_EXT_EXPONENTIAL
+            rng.d_q = qd.data_ptr()
+        else:
+            rng.mode = _lib.RNG_PHILOX
+        opts = GenOpts()
+        opts.kernel = _lib.KERNELS[kernel]
+        opts.mu_law = 1 if mu_law else 0
+        opts.max_steps = int(max_steps)
+        if fold is not None:
+            opts.fold_target, opts.fold_overlap = int(fold[0]), int(fold[1])
+        pk_u = pk_s = None
+        if pack is not None:
+            pk_u = torch.as_tensor(np.ascontiguousarray(pack['utt'], dtype=np.int32)).to(dev)
+            pk_s = torch.as_tensor(np.ascontiguousarray(pack['start'], dtype=np.int32)).to(dev)
+            rows, segs = pk_u.shape
+            if tuple(pk_s.shape) != (rows, segs + 1) or rows != int(pack['rows']):
+                raise ValueError('pack: utt must be [rows, segs], start [rows, segs + 1]')
+            opts.d_pack_utt, opts.d_pack_start = pk_u.data_ptr(), pk_s.data_ptr()
+            opts.pack_rows, opts.pack_segs, opts.pack_steps = rows, segs, int(pack['steps'])
+        uf = None
+        if utt_frames is not None:
+            uf = torch.as_tensor(utt_frames).to(device=dev, dtype=torch.int32).contiguous()
+            if tuple(uf.shape) != (B,):
+                raise ValueError('utt_frames must be [B]')
+            opts.d_utt_frames = uf.data_ptr()
+        td = None
+        if teacher is not None:
+            td = torch.as_tensor(teacher).to(device=dev, dtype=torch.int16).contiguous()
+            if tuple(td.shape) != (GB, GS):
+                raise ValueError('teacher must be [B, S] ([n_folds, fold_len] when folding)')
+            opts.d_teacher = td.data_ptr()
+        logits = None
+        if return_logits:
+            logits = torch.empty(steps, GB, self.n_classes, device=dev, dtype=torch.float32)
+            opts.d_logits = logits.data_ptr()
+        return rng, opts, [t for t in (qd, td, uf, ids, pk_u, pk_s) if t is not None], logits
+
+    def generate_stream(self, mels, *, seed: int = 0, utterance_offset: int = 0, utterance_ids=None, utt_frames=None,
+                        mu_law: bool = True, q=None, teacher=None, chunk_steps: int | None = None, timeout_s: float = 30.0,
+                        device_out: dict | None = None):
+        """Generator: the wave of `generate` (same arguments, same bits) handed out WHILE the push kernel runs.
+
+        Yields (start, chunk): chunk is a float64 numpy array [B, n] of the final samples [start, start + n) of every row, in
+        order, until all (T-1)*hop samples have been yielded; a chunk is ready every `chunk_steps` lock-steps (default: one
+        hop = one mel frame, 12.5 ms of audio).  1..32 rows, PHILOX or external noise; no folding / packing / max_steps.
+        The launch happens at the first next().  Raises if the kernel gives up, if no progress is seen for `timeout_s`, or if
+        the final check() fails.  A consumer that stops early still waits (on close) until the launch has finished writing the
+        pinned buffers this generator owns.  device_out (a dict), if given, receives the call's device `labels` and `wave`.
+        """
+        m = self._mel(mels)
+        B, _, T = m.shape
+        S, L = T * self.hop, (T - 1) * self.hop
+        chunk = self.hop if chunk_steps is None else int(chunk_steps)
+        if chunk < 1:
+            raise ValueError('chunk_steps must be >= 1')
+        dev = self._dev()
+        stream = torch.cuda.current_stream(self.device)
+        with torch.cuda.device(self.device):
+            labels = torch.zeros(B, S, device=dev, dtype=torch.int16)
+            wave = torch.empty(B, L, device=dev, dtype=torch.float64)
+            h_wave = torch.empty(B, L, dtype=torch.float64, pin_memory=True)
+            h_prog = torch.zeros(1, dtype=torch.int64, pin_memory=True)
+            rng, opts, keep, _ = self._call_args(B, B, S, S, seed=seed, utterance_offset=utterance_offset,
+                                                 utterance_ids=utterance_ids, q=q, teacher=teacher, return_logits=False,
+                                                 mu_law=mu_law, kernel='auto', max_steps=0, fold=None, utt_frames=utt_frames,
+                                                 pack=None)
+            _lib.check(self.lib.b200tts_wavernn_generate_stream(
+                self._h, _ptr(m), B, T, C.byref(rng), C.byref(opts), chunk, C.c_void_p(h_wave.data_ptr()),
+                C.c_void_p(h_prog.data_ptr()), _ptr(labels), _ptr(wave), C.c_void_p(stream.cuda_stream)))
+        if device_out is not None:
+            device_out.update(labels=labels, wave=wave)
+        hw = h_wave.numpy()
+        seen = C.c_int64()
+        done, finished = 0, False
+        try:
+            while done < L:
+                want = min(L, done + chunk)              # sample n is final once progress > n
+                _lib.check(self.lib.b200tts_wavernn_stream_wait(C.c_void_p(h_prog.data_ptr()), want, int(timeout_s * 1000),
+                                                                C.byref(seen)))
+                p = int(seen.value)
+                if p < 0:
+                    self.check()                         # raises with the kernel's own message
+                    raise _lib.B200TTSError(-2, 'streaming kernel gave up (a peer thread block did not answer)')
+                if p < want:
+                    raise TimeoutError(f'no streaming progress for {timeout_s} s (at {p} of {L} samples)')
+                n = min(p, L)
+                yield done, hw[:, done:n].copy()
+                done = n
+            self.check()
+            finished = True
+        finally:
+            if not finished:
+                stream.synchronize()                     # the kernel may still write h_wave / h_prog: never free them under it
+            del keep, m, h_wave, h_prog
 
     def fold_geometry(self, T: int, target: int, overlap: int):
         """(n_folds, fold_len) of fold_with_overlap for a T-frame utterance."""

@@ -173,3 +173,19 @@ def synthesize_sharded(synth, wavernn_engine, texts, seed=0, group=None, kernel=
         for k, i in enumerate(share):
             out[i] = host[k, :lens[i]].copy()
     return out, list(mels)
+
+
+def synthesize_stream(synth, wavernn_engine, text, seed=0, utterance_offset=0, chunk_steps=None):
+    """Text -> audio for ONE sentence, handed out while the vocoder runs: Tacotron decodes the whole mel first, then the
+    push kernel streams the wave (WaveRNNEngine.generate_stream).  Yields (start, float64 chunk [n]) until the sentence's
+    (max(T, 21) - 1) * hop samples are out; concatenated they are bit for bit synthesize_batch(synth, eng, [text])[0][0]
+    (same noise key: the sentence is global utterance `utterance_offset`, padded to MIN_FRAMES like vocode_ragged)."""
+    mels, _ = synth.mels([text], seed=seed, utterance_offset=utterance_offset)
+    mel = mels[0]
+    frames = int(mel.shape[0])
+    T = max(frames, MIN_FRAMES)
+    batch = np.zeros((1, mel.shape[1], T), dtype=np.float32)
+    batch[0, :, :frames] = mel.T
+    for start, chunk in wavernn_engine.generate_stream(torch.as_tensor(batch), seed=seed, utterance_ids=[int(utterance_offset)],
+                                                       utt_frames=np.array([T], dtype=np.int32), chunk_steps=chunk_steps):
+        yield start, chunk[0]
